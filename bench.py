@@ -2,6 +2,7 @@
 """bench.py -- simulated request-completions/s of the replica engine (driver contract).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c3|c2|c4|c5]
+                    [--dump-outputs DIR]
 
 Default workload (BASELINE.json configs[2], the one the north-star target is quoted on):
 client -> LB -> {srv-1, srv-2} (README dashboard example), 100 000 replicas per GPU,
@@ -18,6 +19,10 @@ BASELINE shapes (configs[1], [3], [4]); see WORKLOADS below.
             ids, hence its own random numbers): equal work per rank by construction, no traffic during
             simulation, one NCCL all-gather of each rank's summary block (reduced latency histogram +
             totals) per step.
+
+`--dump-outputs DIR` writes, after the timed steps, what the last one handed its caller as
+DIR/<name>.npy (float64; see dump_outputs), so two builds can be compared output for output: with the
+same arguments the inputs are the same in every run.
 
 `--impl reference` times the reference's CPU path (oracle/des_port.py: the actor
 generators on a simpy-4.1.1-compatible heap, restated because simpy is not installable
@@ -364,6 +369,36 @@ def profiled(config_key: str) -> dict:
     return {}
 
 
+# --------------------------------------------------------------------------- outputs
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, res) -> None:
+    """The last end-to-end step's results (SweepRunner.collect's per-replica arrays and the all-gathered
+    summary) as float64 DIR/<name>.npy, at most DUMP_BYTES in all: past that, every per-replica array keeps
+    the same fixed, seeded sample of rows, and replica_rows.npy names them (this rank's rows)."""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    g = res.global_summary
+    whole = {"summary_histogram": g.histogram,
+             "summary_counts": np.array([g.completed, g.generated, g.events, g.replicas, g.overflowed]),
+             "summary_latency": np.array([g.lat_sum, g.lat_min, g.lat_max])}
+    per_replica = {f"stats_{f}": res.stats[f] for f in res.stats.dtype.names}
+    per_replica.update(edge_sent=res.edge_sent, edge_dropped=res.edge_dropped,
+                       sampled_sum=res.samp_sum, sampled_max=res.samp_max)
+    if res.throughput is not None:
+        per_replica["throughput"] = res.throughput
+    n = len(res)
+    row_bytes = 8 + sum(8 * int(np.prod(a.shape[1:])) for a in per_replica.values())        # + replica_rows
+    budget = DUMP_BYTES - sum(8 * a.size for a in whole.values()) - 256 * (len(whole) + len(per_replica) + 1)
+    rows = np.arange(n)
+    if n * row_bytes > budget:
+        rows = np.sort(np.random.default_rng(SEED).choice(n, budget // row_bytes, replace=False))
+    out = {**whole, **{k: a[rows] for k, a in per_replica.items()}, "replica_rows": rows}
+    for name, a in out.items():
+        np.save(d / f"{name}.npy", np.asarray(a, dtype=np.float64))
+
+
 # --------------------------------------------------------------------------- arms
 def run_reference(a) -> None:
     rank = int(os.environ.get("RANK", "0"))
@@ -519,6 +554,9 @@ def run_ours(a) -> None:
             dist.destroy_process_group()
         return
 
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, res)
+
     value = completed * a.steps / (dev_ms / 1e3)
     e2e_value = completed * a.steps / wall_e2e
     peak, peak_src = hbm_peak()
@@ -610,7 +648,13 @@ def main() -> None:
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--e2e-warm", type=int, default=1, help="0: no untimed end-to-end step before the timed ones (the first timed "
                     "one then also allocates the pinned result buffers; for the multi-minute BASELINE-size runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's results to DIR/<name>.npy (float64, at most 64 MB)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the results of the engine (--impl ours)")
     a.warmup = max(a.warmup, 0)
     claim_stdout()
     try:

@@ -28,7 +28,7 @@ here                         reference (``/root/reference/src/asyncflow``)
 ``simulate`` (start order)   runtime/simulation_runner.py:349-376, 301-342
 ===========================  ==================================================
 
-Parity pin: ``tests/test_oracle.py`` (build container: needs /root/reference) requires
+Parity pin: ``tests/test_oracle.py`` (against the stored reference runs) requires
 this port to reproduce ``ref_harness.run_reference`` -- the unmodified
 reference actors -- bit for bit (every (start, finish) clock, every counter,
 every sampled series) on all scenarios under ``tests/scenarios``; the golden

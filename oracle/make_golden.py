@@ -1,8 +1,8 @@
 """Generate tests/golden/*.json from the UNMODIFIED reference actors.
 
-Run in the build container (needs /root/reference):
+Needs a checkout of the reference:
 
-    python oracle/make_golden.py
+    ASYNCFLOW_REFERENCE_SRC=<reference>/src python oracle/make_golden.py
 
 Every vector is one replica of a scenario under tests/scenarios, simulated by
 ``oracle/ref_harness.run_reference`` -- the reference's own ``SimulationRunner``
@@ -90,7 +90,7 @@ def vector(payload: dict, replica: int) -> dict:
 
 def main(only_full: bool = False) -> None:
     if not ref_harness.reference_available():
-        sys.exit("needs /root/reference")
+        sys.exit("set ASYNCFLOW_REFERENCE_SRC to the src/ directory of a reference checkout")
     gold = ROOT / "tests" / "golden"
     gold.mkdir(exist_ok=True)
     for name, (horizon, replicas) in ({} if only_full else CASES).items():

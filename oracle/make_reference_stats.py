@@ -1,6 +1,6 @@
 """Statistics of the UNMODIFIED reference with its OWN RNG (numpy PCG64) -> tests/golden/.
 
-    python oracle/make_reference_stats.py            # build container only (/root/reference)
+    ASYNCFLOW_REFERENCE_SRC=<reference>/src python oracle/make_reference_stats.py
 
 The bit-exact parity chain (ref_harness -> des_port -> engine) injects AF-RNG through the
 reference's seeding seam.  This script is the independent, statistical leg: the reference runs
@@ -48,7 +48,7 @@ def one(payload_dict: dict, seed: int) -> dict:
 
 def main() -> None:
     if not ref_harness.reference_available():
-        sys.exit("needs /root/reference")
+        sys.exit("set ASYNCFLOW_REFERENCE_SRC to the src/ directory of a reference checkout")
     out = {}
     for name, (horizon, n) in CASES.items():
         payload = yaml.safe_load((ROOT / "tests" / "scenarios" / name).read_text())

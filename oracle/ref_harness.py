@@ -1,9 +1,10 @@
 """Run the UNMODIFIED reference actors on the oracle kernel with AF-RNG injected.
 
-ORACLE / TEST INFRASTRUCTURE ONLY.  Needs ``/root/reference`` (build container
-only -- it does not exist on the GPU box); its job is to (a) pin
-``oracle/des_port.py`` to the real reference code and (b) generate the golden
-vectors committed under ``tests/golden/`` (``oracle/make_golden.py``).
+ORACLE / TEST INFRASTRUCTURE ONLY.  Needs a checkout of the reference, its ``src/``
+directory named by ``ASYNCFLOW_REFERENCE_SRC``; its job is to generate the golden
+data committed under ``tests/golden/`` (``oracle/make_golden.py``,
+``oracle/make_reference_runs.py``), which pins ``oracle/des_port.py`` and the
+engine to the real reference code.
 
 What is "unmodified": every class under ``/root/reference/src/asyncflow`` is
 imported and executed as shipped -- ``SimulationRunner.run()``
@@ -24,12 +25,13 @@ exactly as upstream.  Three seams are used, none edits reference source:
 
 from __future__ import annotations
 
+import os
 import sys
 import types
 from pathlib import Path
 
 _HERE = Path(__file__).resolve().parent
-REFERENCE_SRC = Path("/root/reference/src")
+REFERENCE_SRC = Path(os.environ.get("ASYNCFLOW_REFERENCE_SRC", "")).resolve()
 
 if str(_HERE) not in sys.path:
     sys.path.insert(0, str(_HERE))
@@ -38,7 +40,7 @@ import afrng  # noqa: E402
 
 
 def reference_available() -> bool:
-    return (REFERENCE_SRC / "asyncflow" / "__init__.py").exists()
+    return bool(os.environ.get("ASYNCFLOW_REFERENCE_SRC")) and (REFERENCE_SRC / "asyncflow" / "__init__.py").is_file()
 
 
 def _ensure_paths() -> None:

@@ -17,7 +17,6 @@ SEED = 0xA5F10
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (B200); run with -m gpu")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only)")
 
 
 def pytest_collection_modifyitems(config, items):

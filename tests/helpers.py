@@ -9,6 +9,8 @@ from pathlib import Path
 import numpy as np
 import yaml
 
+from asyncflow_b200 import _capi as K
+
 ROOT = Path(__file__).resolve().parent.parent
 SCEN = ROOT / "tests" / "scenarios"
 GOLD = ROOT / "tests" / "golden"
@@ -37,6 +39,46 @@ def load_golden(name: str) -> dict:
 
 def sha(arr: np.ndarray) -> str:
     return hashlib.sha256(np.ascontiguousarray(arr).tobytes()).hexdigest()
+
+
+def f64_digest(values) -> str:
+    """SHA-256 of ``values`` as little-endian f64: how tests/golden/reference_runs.json pins clock lists
+    and sampled series."""
+    return sha(np.asarray(values, dtype="<f8"))
+
+
+def load_reference_runs() -> dict:
+    """What the unmodified reference computed for the reference-comparison tests
+    (oracle/make_reference_runs.py)."""
+    return json.loads((GOLD / "reference_runs.json").read_text())
+
+
+def assert_matches_reference_run(rec: dict, *, generated, completed, clocks, edge_sent, edge_dropped,
+                                 server_series=None, edge_series=None) -> None:
+    """One run against one record of reference_runs.json, bit for bit; every series the reference
+    sampled must be there (``*_series``: {entity id: {metric: list}})."""
+    assert generated == rec["generated"]
+    assert completed == rec["completed"]
+    assert dict(edge_sent) == rec["edge_sent"]
+    assert dict(edge_dropped) == rec["edge_dropped"]
+    assert f64_digest(clocks) == rec["clocks_sha256"]
+    for got, key in ((server_series, "server_series"), (edge_series, "edge_series")):
+        if got is None:
+            continue
+        for ent, per in rec[key].items():
+            for m, dig in per.items():
+                assert f64_digest(got[ent][m]) == dig, (ent, m)
+
+
+def pod_tables(flat) -> list[bytes]:
+    """The flattened scenario as bytes, pointers left out: the header and every table row."""
+    p = flat.pod
+    out = [bytes(p)[: K.AfScenario.edges.offset]]
+    for arr, n in (("edges", p.n_edges), ("servers", p.n_servers), ("endpoints", p.n_endpoints),
+                   ("steps", p.n_steps), ("spike_marks", p.n_spike_marks), ("outage_marks", p.n_outage_marks)):
+        out += [bytes(getattr(p, arr)[i]) for i in range(n)]
+    out.append(np.array([p.lb_edges[i] for i in range(p.n_lb_edges)], dtype="<i4").tobytes())
+    return out
 
 
 def unhex(pairs) -> np.ndarray:

@@ -81,3 +81,39 @@ def test_effective_cores_respects_affinity_and_quota():
     assert 1 <= n <= (info["os_cpu_count"] or 1) and n <= info["affinity"]
     if info["cgroup_quota_cpus"]:
         assert n <= max(1, round(info["cgroup_quota_cpus"]))
+
+
+def test_dump_outputs_writes_the_results_as_float64_within_the_budget(tmp_path, monkeypatch):
+    """--dump-outputs on results of the twin-backed SweepRunner: every array float64, the per-replica ones
+    whole while they fit, one fixed sample of rows (the same in every run) once they do not."""
+    import numpy as np
+    from twin_engine import TwinEngine
+
+    import asyncflow_b200.runner as R
+    import bench
+    from asyncflow_b200 import flatten
+    from asyncflow_b200.distributed import all_gather_summary, summary_block
+    monkeypatch.setattr(R, "Engine", TwinEngine)
+    w = bench.make_workload("c3", horizon=3, replicas=40)
+    flat = flatten(w.payload)
+    sw = R.SweepRunner(flat, 40, w.columns(flat, np.arange(40), 40), seed=bench.SEED, pinned=False)
+    res = sw.run()
+    res.global_summary = all_gather_summary(*summary_block(res.stats, None))
+
+    bench.dump_outputs(str(tmp_path / "all"), res)
+    got = {p.stem: np.load(p) for p in (tmp_path / "all").glob("*.npy")}
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert np.array_equal(got["replica_rows"], np.arange(40))
+    assert np.array_equal(got["stats_completed"], res.stats["completed"])
+    assert np.array_equal(got["sampled_sum"], res.samp_sum) and np.array_equal(got["edge_dropped"], res.edge_dropped)
+    assert got["summary_counts"][0] == res.stats["completed"].sum()
+
+    monkeypatch.setattr(bench, "DUMP_BYTES", 48 << 10)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), res)
+        assert sum(p.stat().st_size for p in (tmp_path / run).glob("*.npy")) <= bench.DUMP_BYTES
+    rows = np.load(tmp_path / "a" / "replica_rows.npy").astype(np.int64)
+    assert 0 < len(rows) < 40 and np.all(np.diff(rows) > 0)
+    assert np.array_equal(np.load(tmp_path / "a" / "stats_lat_sum.npy"), res.stats["lat_sum"][rows])
+    for p in (tmp_path / "a").glob("*.npy"):
+        assert p.read_bytes() == (tmp_path / "b" / p.name).read_bytes(), p.name

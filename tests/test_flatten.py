@@ -4,9 +4,8 @@ from __future__ import annotations
 
 import numpy as np
 import pytest
-from helpers import load_scenario
+from helpers import load_reference_runs, load_scenario, pod_tables
 
-import ref_harness
 from asyncflow_b200 import _capi as K
 from asyncflow_b200.flatten import SweepSpec, flatten
 
@@ -117,18 +116,10 @@ def test_sweep_runner_hands_out_payloads_without_a_device():
         SweepRunner(flatten(base), 2, pinned=False).payload_for(0)
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not ref_harness.reference_available(), reason="/root/reference not on this box")
 @pytest.mark.parametrize("name", ["c1_my_service.yml", "c4_lb8_events.yml", "mixed_lc.yml", "ev_spikes_outages.yml"])
 def test_validated_payload_flattens_like_the_raw_dict(name):
-    ref_harness._ensure_paths()
-    from asyncflow.schemas.payload import SimulationPayload
+    """The schema defaults flatten() fills in are the reference's: the raw YAML dict flattens like the
+    reference's own SimulationPayload validation of it (stored as its model_dump)."""
     d = load_scenario(name)
-    a, b = flatten(d), flatten(SimulationPayload.model_validate(d))
-    assert bytes(a.pod)[: K.AfScenario.edges.offset] == bytes(b.pod)[: K.AfScenario.edges.offset]
-    for arr, n in (("edges", a.pod.n_edges), ("servers", a.pod.n_servers), ("endpoints", a.pod.n_endpoints),
-                   ("steps", a.pod.n_steps), ("spike_marks", a.pod.n_spike_marks),
-                   ("outage_marks", a.pod.n_outage_marks)):
-        for i in range(n):
-            assert bytes(getattr(a.pod, arr)[i]) == bytes(getattr(b.pod, arr)[i]), (arr, i)
-    assert [a.pod.lb_edges[i] for i in range(a.pod.n_lb_edges)] == [b.pod.lb_edges[i] for i in range(b.pod.n_lb_edges)]
+    validated = load_reference_runs()["validated_payloads"][name]
+    assert pod_tables(flatten(d)) == pod_tables(flatten(validated))

@@ -1,23 +1,21 @@
-"""The OUT seam: engine results fed to the reference's REAL ResultsAnalyzer.
+"""The OUT seam: engine results against what the reference's REAL ResultsAnalyzer computed.
 
-Needs /root/reference (build container, no GPU), so the engine results come from the CPU
-debugging twin; the object under test is the product's `ReplicaResults` (holders, getters,
-`to_reference_analyzer`).  On the GPU box the same class is exercised with real engine output
-by tests/test_gpu_parity.py::test_runner_api_mirrors_the_reference."""
+The reference side is tests/golden/reference_runs.json (oracle/make_reference_runs.py: the unmodified
+reference actors and analyzer), the engine side comes from the CPU debugging twin; the object under
+test is the product's `ReplicaResults` (holders, getters).  On the GPU the same class is exercised with
+real engine output by tests/test_gpu_parity.py::test_runner_api_mirrors_the_reference."""
 
 from __future__ import annotations
 
-import numpy as np
+import des_port
 import pytest
 import twin
-from helpers import SEED, load_scenario
+from helpers import SEED, assert_matches_reference_run, f64_digest, load_reference_runs, load_scenario
 
-import ref_harness
 from asyncflow_b200.flatten import flatten
 from asyncflow_b200.results import ReplicaResults
 
-pytestmark = [pytest.mark.reference,
-              pytest.mark.skipif(not ref_harness.reference_available(), reason="/root/reference not on this box")]
+REFERENCE_RUNS = load_reference_runs()
 
 
 def twin_results(payload, replica) -> ReplicaResults:
@@ -31,39 +29,49 @@ def twin_results(payload, replica) -> ReplicaResults:
                           n_events=int(st["n_events"]), flags=int(st["flags"]))
 
 
+def assert_sampled(rec: dict, got: dict) -> None:
+    """Every series the reference analyzer holds, bit for bit (``rec``: {metric: {entity: digest}})."""
+    assert set(rec) == set(got)
+    for metric in rec:
+        assert set(rec[metric]) == set(got[metric])
+        for ent, dig in rec[metric].items():
+            assert f64_digest(got[metric][ent]) == dig, (metric, ent)
+
+
 @pytest.mark.parametrize("name,horizon", [("c1_my_service.yml", 15), ("ev_spikes_outages.yml", None), ("mixed_lc.yml", None)])
 def test_reference_analyzer_on_engine_results_equals_reference_run(name, horizon):
-    payload = load_scenario(name, horizon)
-    ref = ref_harness.run_reference(payload, seed=SEED, replica=4)
-    mine = twin_results(payload, 4)
-    ra, rb = ref["analyzer"], mine.to_reference_analyzer()       # both are asyncflow ResultsAnalyzer
-    assert type(ra) is type(rb)
-    sa, sb = ra.get_latency_stats(), rb.get_latency_stats()
-    assert {k.value: v for k, v in sa.items()} == {k.value: v for k, v in sb.items()}
-    assert ra.get_throughput_series() == rb.get_throughput_series()
-    assert ra.get_throughput_series(window_s=2.5) == rb.get_throughput_series(window_s=2.5)
-    ma, mb = ra.get_sampled_metrics(), rb.get_sampled_metrics()
-    assert set(ma) == set(mb)
-    for metric in ma:
-        assert set(ma[metric]) == set(mb[metric])
-        for ent in ma[metric]:
-            assert list(ma[metric][ent]) == list(mb[metric][ent]), (metric, ent)
-    assert ra.list_server_ids() == rb.list_server_ids()
+    rec = REFERENCE_RUNS["analyzer"][name]
+    mine = twin_results(load_scenario(name, horizon), 4)
+    assert f64_digest(mine.clocks) == rec["clocks_sha256"]
+    # what ResultsAnalyzer reads through its duck-typed seam
+    h = mine.holders()
+    assert f64_digest([(c.start, c.finish) for c in h["client"].rqs_clock]) == rec["clocks_sha256"]
+    held: dict = {}
+    for s in h["servers"]:
+        for k, v in s.enabled_metrics.items():
+            held.setdefault(k.value, {})[s.server_config.id] = v
+    for e in h["edges"]:
+        for k, v in e.enabled_metrics.items():
+            held.setdefault(k.value, {})[e.edge_config.id] = v
+    assert_sampled(rec["sampled"], held)
+    assert (h["settings"].total_simulation_time, h["settings"].sample_period_s) == (mine.flat.horizon_s, mine.flat.sample_period)
     # and the product's own getters agree with the reference analyzer's
-    own = mine.get_latency_stats()
-    assert own == {k.value: v for k, v in sa.items()}
-    assert mine.get_throughput_series() == ra.get_throughput_series()
-    t_a, v_a = ra.get_series("ram_in_use", mine.flat.server_ids[0])
-    t_b, v_b = mine.get_series("ram_in_use", mine.flat.server_ids[0])
-    assert v_a == v_b and np.allclose(t_a, t_b)
-    assert mine.format_latency_stats() == ra.format_latency_stats()
+    assert mine.get_latency_stats() == rec["latency_stats"]
+    assert [list(x) for x in mine.get_throughput_series()] == rec["throughput"]
+    assert [list(x) for x in mine.get_throughput_series(window_s=2.5)] == rec["throughput_2_5"]
+    assert_sampled(rec["sampled"], mine.get_sampled_metrics())
+    assert mine.list_server_ids() == rec["server_ids"]
+    ser = rec["ram_in_use_series"]
+    t, v = mine.get_series("ram_in_use", ser["server"])
+    assert (f64_digest(t), f64_digest(v)) == (ser["t"], ser["v"])
+    assert mine.format_latency_stats() == rec["format_latency_stats"]
 
 
 @pytest.mark.parametrize("seed", [301, 305, 312, 327])
 def test_sweep_row_equals_unmodified_reference_on_payload_for(seed):
-    """A sweep point handed back to the reference: SweepSpec.payload_for(i) passes the reference's
-    own SimulationPayload validation, and the UNMODIFIED reference actors run on it produce the
-    clocks the engine produced for row i of the sweep."""
+    """A sweep point handed back to the reference: the UNMODIFIED reference actors, run on
+    SweepSpec.payload_for(i), produced the clocks the engine produces for row i of the sweep; the port
+    (pinned to those actors by tests/test_oracle.py) reproduces them from today's payload_for(i)."""
     import fuzz
 
     from asyncflow_b200.flatten import SweepSpec
@@ -74,12 +82,13 @@ def test_sweep_row_equals_unmodified_reference_on_payload_for(seed):
     spec = SweepSpec(flat, n, fuzz.sweep_columns(seed, payload, n))
     r = twin.run(flat, seed=SEED, replica_begin=0, n=n, sweep=spec, trace=n, clock_cap=100000, request_capacity=200000)
     for i in range(n):
-        p = spec.payload_for(payload, i)
-        ref = ref_harness.run_reference(p, seed=SEED, replica=i)          # validates with the reference schema
+        ref = REFERENCE_RUNS["sweep_rows"][str(seed)][i]
         k = int(r["stats"][i]["completed"])
-        got = [tuple(x) for x in r["trace_clocks"][i, :k].tolist()]
-        assert got == [tuple(w) for w in ref["clocks"]]
+        assert f64_digest(r["trace_clocks"][i, :k]) == ref["clocks_sha256"]
         assert dict(zip(flat.edge_ids, map(int, r["dropped"][i]))) == ref["edge_dropped"]
+        o = des_port.simulate(spec.payload_for(payload, i), seed=SEED, replica=i)
+        assert_matches_reference_run(ref, generated=o["generated"], completed=o["completed"], clocks=o["clocks"],
+                                     edge_sent=o["edge_sent"], edge_dropped=o["edge_dropped"])
 
 
 REFERENCE_YAMLS = ["examples/yaml_input/data/two_servers_lb.yml", "examples/yaml_input/data/event_inj_single_server.yml",
@@ -89,23 +98,14 @@ REFERENCE_YAMLS = ["examples/yaml_input/data/two_servers_lb.yml", "examples/yaml
 
 @pytest.mark.parametrize("rel", REFERENCE_YAMLS)
 def test_every_scenario_file_the_reference_ships_runs_identically(rel):
-    """The reference's own example / test YAMLs, as they lie in /root/reference (read at test time, not
-    copied): unmodified reference actors == engine state machine, clock for clock and series for series."""
-    import yaml
-    from pathlib import Path
-
-    payload = yaml.safe_load((Path(ref_harness.REFERENCE_SRC).parent / rel).read_text())
-    full = int(payload["sim_settings"].get("total_simulation_time", 3600))
-    horizon = min(full, 40)
-    payload["sim_settings"]["total_simulation_time"] = horizon
-    for ev in payload.get("events") or []:                 # same timeline, compressed into the shortened horizon
-        ev["start"]["t_start"] = float(ev["start"]["t_start"]) * horizon / full
-        ev["end"]["t_end"] = float(ev["end"]["t_end"]) * horizon / full
-    ref = ref_harness.run_reference(payload, seed=SEED, replica=2)
-    mine = twin_results(payload, 2)
-    assert [tuple(x) for x in mine.clocks.tolist()] == [tuple(c) for c in ref["clocks"]]
-    assert mine.generated == ref["generated"] and mine.edge_dropped == ref["edge_dropped"]
-    ma, mb = ref["analyzer"].get_sampled_metrics(), mine.get_sampled_metrics()
-    for metric in ma:
-        for ent in ma[metric]:
-            assert list(ma[metric][ent]) == list(mb[metric][ent]), (metric, ent)
+    """The reference's own example / test YAMLs (stored as the payloads run: horizon cut to 40 s, event
+    timeline compressed into it): unmodified reference actors == engine state machine, clock for clock
+    and series for series."""
+    rec = REFERENCE_RUNS["shipped_scenarios"][rel]
+    mine = twin_results(rec["payload"], 2)
+    assert f64_digest(mine.clocks) == rec["clocks_sha256"]
+    assert mine.generated == rec["generated"] and mine.edge_dropped == rec["edge_dropped"]
+    got = mine.get_sampled_metrics()
+    for metric, per in rec["sampled"].items():
+        for ent, dig in per.items():
+            assert f64_digest(got[metric][ent]) == dig, (metric, ent)
